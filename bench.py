@@ -38,6 +38,7 @@ BATCH = 8192                  # rays per GPU of the default configuration (scrip
 UPDATE_INTERVAL = 16          # train.py:57-58
 PREWARM = 20                  # extra untimed steps before the W warm-up steps
 DENSITY_THRESHOLD = 0.01 * 1024 / 3 ** 0.5  # train.py:180
+DUMP_SAMPLE = 1 << 20         # --dump-outputs: hash-table entries written (the full table can exceed 64 MB)
 
 CONFIGS = {
     "lego_fp32_1024": dict(index=0, kind="train", n_rays=1024, half=False, scale=0.5, max_res=1024, esf=0.0,
@@ -152,6 +153,20 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write what the timed path computed in its last step as <out_dir>/<name>.npy (float32, or
+    float64 where the value is float64), so that two builds can be compared output for output on identical inputs.
+    The hash-table gradient is accumulated with atomics, so two runs agree to float-reordering tolerance, not bitwise."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= 64 << 20, total
 
 
 # --------------------------------------------------------------------------------------------------
@@ -319,7 +334,7 @@ def run_train(args, cfg_name, cfg):
             "shadow": None if trainer._shadow_full is None else trainer._shadow_full.clone(),
             "grid": model.density_grid.clone(), "bits": model.density_bitfield.clone(),
             "grid_step": model.__dict__.get("_grid_step", 0), "sample_step": fast.sample_step.clone(),
-            "step_count": trainer.step_count}
+            "step_count": trainer.step_count, "rng": torch.cuda.get_rng_state(dev)}
 
     def restore_state():
         fast.flush()
@@ -337,6 +352,7 @@ def run_train(args, cfg_name, cfg):
         model.__dict__["_grid_step"] = snap["grid_step"]
         fast.sample_step.copy_(snap["sample_step"])
         trainer.step_count = snap["step_count"]
+        torch.cuda.set_rng_state(snap["rng"], dev)   # --path modules: the marching noise comes from torch's RNG
     # untimed pre-warm beyond --warmup: the caching allocator must have seen the range of per-step
     # sample counts (every new size is a cudaMalloc) and the clocks must have ramped up
     step_fn = (lambda i, k: graph_step(i, None)) if use_graph else (lambda i, k: module_step(i, batches[k]))
@@ -361,11 +377,22 @@ def run_train(args, cfg_name, cfg):
     launches0 = _lib.launch_count()
     graph0 = fast.graph_kernel_launches
 
+    last_loss = []
+
     def timed_steps():
         for k in range(args.steps):
-            step_fn(args.warmup + k, args.warmup + k)
+            last_loss[:] = [step_fn(args.warmup + k, args.warmup + k)]
         fast.flush()   # every one of the K updates is applied inside the timed region
     ms_total = timed(timed_steps)
+    if args.dump_outputs and rank == 0:
+        # the step's loss and the parameters it leaves (a fixed, seeded sample of the hash table, all MLP weights)
+        P = model.pos_encoder.total_param_size
+        pick = np.sort(np.random.default_rng(SEED).choice(P, min(P, DUMP_SAMPLE), replace=False))
+        dump_outputs(args.dump_outputs, {
+            "loss": last_loss[0].detach().float().reshape(1).cpu().numpy(),
+            "samples": sample_counts[-1].reshape(1).cpu().numpy().astype(np.float64),
+            "hash_table_sample": trainer.flat_param[torch.from_numpy(pick).to(dev)].cpu().numpy(),
+            "mlp_params": trainer.flat_param[P:].cpu().numpy()})
     trainer.p2p_check()   # (several ranks) no peer barrier gave up waiting
     clock_info = clocks.stop() if rank == 0 else None
     launches = _lib.launch_count() - launches0            # eager launches of libngp_b200 kernels
@@ -616,7 +643,11 @@ def run_frame(args, cfg_name, cfg):
         res = frame(pose)
         k += 1
     launches0 = _lib.launch_count()
-    ms = timed(lambda: [frame(pose) for _ in range(args.steps)]) / args.steps
+    timed_frames = []
+    ms = timed(lambda: timed_frames.extend(frame(pose) for _ in range(args.steps))) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: timed_frames[-1][k].float().cpu().numpy() for k in ("rgb", "depth", "opacity")})
+    del timed_frames
     launches = _lib.launch_count() - launches0
     clock_info = clocks.stop()
     total_samples = int(res["total_samples"])
@@ -917,7 +948,13 @@ def main():
     ap.add_argument("--ncu-window", type=int, default=0,
                     help="profiling aid: wrap this many extra steps in cudaProfilerStart/Stop "
                          "(use with `ncu --profile-from-start off`); numbers printed under ncu are not bench values")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy "
+                         "(train: loss, sample count, a seeded sample of the hash table, MLP weights; frame: rgb, "
+                         "depth, opacity), at most 64 MB")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.ncu_window > 0):
+        ap.error("--dump-outputs applies to the timed CUDA path only")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     cfg = CONFIGS[args.config]

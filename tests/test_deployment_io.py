@@ -76,17 +76,28 @@ def test_deployment_npy_and_bin_round_trip(tmp_path):
         load_deployment_model(NGP(scale=0.5), blob)                            # stock architecture: shapes differ
 
 
-REF = "/root/reference/deployment/InstantNGP/taichi_ngp/compiled"
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "hash_embedding.bin")), reason="reference checkout not available")
-def test_shipped_lego_files_load_into_the_model():
+def test_shipped_lego_files_load_into_the_model(tmp_path):
+    """A folder of .bin files in the reference's container format: the small files are the shipped ones byte for byte,
+    the table and the bitfield carry the shipped headers over the stored part of the model (oracle/kat_lego.py), and
+    directions.bin holds the stored view's camera directions (a subsample of the shipped file) under its own header."""
     from modules.networks import NGP
     from modules.utils import load_deployment_model, read_aot_array
+    from oracle import kat_lego
+    P = kat_lego.load_part()
+    z = P["raw"]
+    head = {str(n): h for n, h in zip(z["bin_names"], z["bin_headers"])}
+    payload = {"sigma_weights": z["sigma_weights_bin"][8:], "rgb_weights": z["rgb_weights_bin"][8:],
+               "pose": z["pose_bin"][8:], "hash_embedding": P["table"], "density_bitfield": P["bits"]}
+    for n, a in payload.items():
+        with open(tmp_path / (n + ".bin"), "wb") as f:
+            f.write(head[n].astype(np.int32).tobytes() + np.ascontiguousarray(a).tobytes())
+    with open(tmp_path / "directions.bin", "wb") as f:
+        f.write(np.array([head["directions"][0], P["directions"].size], np.int32).tobytes() + P["directions"].tobytes())
     m = NGP(**DEPLOY_CFG)
-    extra = load_deployment_model(m, REF)
-    assert extra['pose'].size == 12 and extra['model.directions'].size == 600 * 300 * 3
-    emb = read_aot_array(os.path.join(REF, "hash_embedding.bin"))
+    extra = load_deployment_model(m, str(tmp_path))
+    assert extra['pose'].size == 12 and np.array_equal(extra['pose'].reshape(3, 4), P["pose"])
+    assert np.array_equal(extra['model.directions'], P["directions"].reshape(-1))
+    emb = read_aot_array(str(tmp_path / "hash_embedding.bin"))
     assert torch.equal(m.pos_encoder.hash_table.detach().reshape(-1), torch.from_numpy(emb.copy()))
-    from conftest import GOLDEN
-    assert np.array_equal(m.density_bitfield.numpy(), np.load(os.path.join(GOLDEN, "lego_bitfield.npz"))["bitfield"])
+    assert np.array_equal(m.density_bitfield.numpy(), P["bits"])
+    assert torch.equal(m.xyz_encoder.hidden_layers[0].weight.detach().reshape(-1), torch.from_numpy(P["sigma_w"][:256]))

@@ -286,25 +286,27 @@ def test_static_step_with_device_sampled_batches(lego_bitfield, use_graph):
         assert int(fs1.sample_step) == 3
 
 
-def test_shipped_lego_model_renders_on_gpu():
-    """Known-answer test on the CUDA path: the reference's shipped, trained Lego deployment model (L=4 F=4 dense
-    grid, 16-wide MLPs; staged under oracle/_ref/ by __graft_entry__.build()) loaded with load_deployment_model and
-    rendered through render(test_time=True) must reproduce the oracle's golden image of the same rays
-    (tests/golden/lego_kat.png, made by oracle/kat_lego.py)."""
-    import os
-    import __graft_entry__ as g
-    from conftest import GOLDEN
-    if not g.stage_lego_fixture():
-        pytest.skip("shipped Lego weights not staged (needs one build() in the container that has /root/reference)")
-    from PIL import Image
+def _shipped_lego_part():
+    """The stored part of the reference's shipped, trained Lego deployment model (L=4 F=4 dense grid, 16-wide MLPs;
+    oracle/kat_lego.py) as an NGP on the GPU, and the part's other fixture arrays."""
     from modules.networks import NGP
-    from modules.rendering import render
     from modules.utils import load_deployment_model
+    from oracle import kat_lego
+    P = kat_lego.load_part()
     model = NGP(scale=0.5, pos_encoder_type='hash', levels=4, feature_per_level=4, base_res=32, max_res=128,
                 log2_T=21, xyz_net_width=16, rgb_net_width=16, rgb_net_depth=1).cuda()
-    extra = load_deployment_model(model, g.LEGO_FIXTURE)
-    pose = torch.from_numpy(extra['pose'].reshape(3, 4).copy()).cuda()
-    directions = torch.from_numpy(extra['model.directions'].reshape(600, 300, 3)[::2, ::2].copy()).cuda()
+    load_deployment_model(model, P["blob"])
+    return model.eval(), P
+
+
+def test_shipped_lego_model_renders_on_gpu():
+    """Known-answer test on the CUDA path: the part of the reference's shipped, trained Lego deployment model loaded
+    with load_deployment_model and rendered through render(test_time=True) must reproduce the oracle's golden image of
+    the same rays (made with the full shipped table, tests/golden/make_golden.py)."""
+    from modules.rendering import render
+    model, P = _shipped_lego_part()
+    pose = torch.from_numpy(P["pose"].copy()).cuda()
+    directions = torch.from_numpy(P["directions"]).cuda()
     h, w = directions.shape[:2]
     dirs = directions.reshape(-1, 3)
     rays_d = dirs @ pose[:, :3].T
@@ -312,13 +314,14 @@ def test_shipped_lego_model_renders_on_gpu():
     with torch.no_grad(), torch.autocast('cuda', dtype=torch.float16):
         out = render(model, rays_o, rays_d, test_time=True, T_threshold=1e-2, exp_step_factor=0.0)
     rgb = out['rgb'].float().reshape(h, w, 3).clamp(0, 1).cpu().numpy()   # render() composites onto white
-    gold = np.asarray(Image.open(os.path.join(GOLDEN, 'lego_kat.png')).convert('RGB'), dtype=np.float32) / 255
+    gold = np.clip(P["gold_rgb"] + (1 - P["gold_opacity"])[..., None], 0, 1)
     assert gold.shape == rgb.shape
     mse = float(((rgb - gold) ** 2).mean())
     psnr = -10 * np.log10(max(mse, 1e-12))
-    assert psnr > 35.0, psnr          # fp16 autocast MLP + 8-bit golden; a layout mistake gives < 15 dB
+    assert psnr > 35.0, psnr          # fp16 autocast MLP; a layout mistake gives < 15 dB
     opacity = out['opacity'].float().reshape(h, w).cpu().numpy()
-    assert 0.55 < float((opacity > 0.5).mean()) < 0.67   # tests/golden/lego_kat_stats.json: coverage 0.611
+    gold_cov = float((P["gold_opacity"] > 0.5).mean())
+    assert abs(float((opacity > 0.5).mean()) - gold_cov) < 0.03, gold_cov
 
 
 @pytest.mark.parametrize("use_graph", [False, True])
@@ -404,17 +407,43 @@ def test_module_path_has_gradscaler_semantics(lego_bitfield):
         tr.optimizer_step()
 
 
+def _teacher_crop_psnr(teacher, model, ds, i, margin=4):
+    """(PSNR of ``model``, PSNR of an all-white image) against the teacher's view ``i`` of ``ds``, both over the crop
+    around the pixels the teacher covers (opacity > 0.01) widened by ``margin`` pixels."""
+    from datasets.ray_utils import get_rays
+    from modules.rendering import render
+    w, h = ds.img_wh
+    td = ds[i]
+    rays_o, rays_d = get_rays(ds.directions, td['pose'])
+    with torch.no_grad(), torch.autocast('cuda', dtype=torch.float16):
+        cover = render(teacher, rays_o, rays_d, test_time=True, T_threshold=1e-2, exp_step_factor=0.0)['opacity']
+        rgb = render(model, rays_o, rays_d, test_time=True)['rgb']      # as train_vs_teacher evaluates
+    cover = cover.float().reshape(h, w) > 0.01
+    rows, cols = torch.nonzero(cover.any(1)).flatten(), torch.nonzero(cover.any(0)).flatten()
+    r0, r1 = max(int(rows[0]) - margin, 0), min(int(rows[-1]) + 1 + margin, h)
+    c0, c1 = max(int(cols[0]) - margin, 0), min(int(cols[-1]) + 1 + margin, w)
+    gt = td['rgb'].reshape(h, w, 3)[r0:r1, c0:c1]
+    rgb = rgb.float().clamp(0, 1).reshape(h, w, 3)[r0:r1, c0:c1]
+    psnr = lambda x: float(-10.0 * torch.log10(((x - gt) ** 2).mean()))   # noqa: E731
+    return psnr(rgb), psnr(torch.ones_like(gt))
+
+
 def test_psnr_vs_teacher():
-    """"PSNR vs ref" protocol (SURVEY.md §8c): the stock fp16 model trained for 1500 graph steps on 200x200 views of the
-    reference's shipped trained Lego model must reach >= 25 dB on held-out teacher views (measured: see
-    profiles/r2_psnr.json; an untrained model scores ~9 dB)."""
-    import __graft_entry__ as g
-    if not g.stage_lego_fixture():
-        pytest.skip("shipped Lego weights not staged (needs one build() in the container that has /root/reference)")
+    """"PSNR vs ref" protocol (SURVEY.md §8c, bench.py's psnr leg: 2000 graph steps on 48 400x400 views): the stock fp16
+    model trained on views of the part of the reference's shipped trained Lego model (the teacher) must reach >= 25 dB
+    on held-out teacher views.  The part covers only a few per cent of a view, so PSNR is taken over the crop around
+    the pixels it covers, where the object fills about as much of the image as the whole model does of a full view:
+    there an all-white image, a model that learned only the background, stays ~16 dB below the gate."""
     from taichi_nerfs_b200.psnr import train_vs_teacher
-    r = train_vs_teacher(torch.device('cuda'), steps=1500, train_views=32, test_views=2, downsample=0.25)
+    teacher, _ = _shipped_lego_part()
+    r = train_vs_teacher(torch.device('cuda'), steps=2000, train_views=48, test_views=2, downsample=0.5,
+                         teacher=teacher)
     assert r is not None
-    assert r["psnr"] >= 25.0, r["psnr_views"]
+    crops = [_teacher_crop_psnr(teacher, r["model"], r["test_dataset"], i) for i in range(len(r["test_dataset"]))]
+    psnr, white = (sum(c[k] for c in crops) / len(crops) for k in (0, 1))
+    print(f"teacher-crop PSNR {psnr:.2f} dB, all-white {white:.2f} dB, whole views {r['psnr']:.2f} dB")
+    assert white < 25.0 - 12.0, crops       # the gate's margin over a trivial answer
+    assert psnr >= 25.0, crops
 
 
 def test_update_density_grid_is_sync_free_and_matches_reference_statistics():
